@@ -75,6 +75,25 @@ def dogman():
     return np.ascontiguousarray(d["src"], dtype=np.float64), np.ascontiguousarray(d["dst"], dtype=np.float64)
 
 
+DUMP_MASK_BYTES = 48 << 20
+
+
+def dump_outputs(dirname, model, mask, stats=None):
+    """Writes what a caller of the timed path receives for its last step, as DIR/<name>.npy, so that two builds can be
+    compared output for output: every pair's model (and stats), its inlier count, and the inlier masks of a fixed,
+    seeded sample of pairs (all of them when they fit in DUMP_MASK_BYTES as float32)."""
+    os.makedirs(dirname, exist_ok=True)
+    P, N = mask.shape
+    k = min(P, DUMP_MASK_BYTES // (4 * N))
+    rows = np.arange(P) if k == P else np.sort(np.random.default_rng(0).choice(P, k, replace=False))
+    out = {"model": model.reshape(P, 3, 3).astype(np.float64), "inliers": mask.sum(1).astype(np.float64),
+           "mask": mask[rows].astype(np.float32), "mask_rows": rows.astype(np.float64)}
+    if stats is not None:
+        out["stats"] = stats.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 # ----------------------------------------------------------------------------- CPU reference arm
 def _cpu_worker(args):
     cfg_id, seed0, count = args
@@ -334,6 +353,13 @@ def run_gpu_arm(args):
         times.append(e0.elapsed_time(e1))
     barrier()
     launches = _cabi.kernel_launches() - launches0
+    dumped = None
+    if args.dump_outputs and rank == 0:     # the last timed step's results, before the legs below run the batch again
+        if world > 1:
+            from pydegensac_b200.parallel import unpack_records
+            dumped = unpack_records(sb.gathered.view(world * P, sb.stride).cpu().numpy())
+        else:
+            dumped = (sb.model.cpu().numpy(), sb.mask.cpu().numpy().astype(bool), sb.stats.cpu().numpy())
     sampler.stop_flag = True        # (its nvidia-smi forks would perturb the host-side e2e leg below)
     sampler.join(2.0)
     total_ms = float(sum(times))
@@ -442,6 +468,8 @@ def run_gpu_arm(args):
                        "reasons": sorted(sampler.reasons)},
         }
         print(json.dumps(line))
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, *dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -463,9 +491,11 @@ def run_latency(args, cfg, dev, rank):
     t0 = time.perf_counter()
     kms = []
     for s in range(args.steps):
+        last = []
         for i in range(calls):
             H, mask = pdg.findHomography(src, dst, cfg["px_th"], cfg["conf"], cfg["max_iters"], seed=1000 + s * calls + i)
             kms.append(_cabi.last_kernel_ms())
+            last.append((H, mask))
     wall = time.perf_counter() - t0
     launches = _cabi.kernel_launches() - launches0
     sampler.stop_flag = True
@@ -495,6 +525,8 @@ def run_latency(args, cfg, dev, rank):
             "gpu_launches": int(launches), "roofline": hbm, "roofline_fp64": None, "cpu_baseline": cpu,
             "clocks": {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": sampler.max_mhz, "reasons": sorted(sampler.reasons)}}
     print(json.dumps(line))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, np.stack([h for h, _ in last]), np.stack([np.asarray(m, bool) for _, m in last]))
 
 
 def main():
@@ -507,7 +539,13 @@ def main():
     ap.add_argument("--pairs-per-gpu", type=int, default=0, help="0 = the config's default")
     ap.add_argument("--cpu-pairs-per-core", type=int, default=0, help="0 = sized per config for ~10-30 s per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU arm")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -6,6 +6,7 @@ libc RNG so the reference can be driven by the engine's Philox sampling stream.
 Only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs may import this.
 """
 import ctypes
+import hashlib
 import os
 
 import numpy as np
@@ -58,6 +59,15 @@ def _declare(_lib):
         _lib.ref_value31.restype = ctypes.c_uint32
         _lib.ref_stateless_sample.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_int, ctypes.c_int,
                                               ctypes.POINTER(ctypes.c_int)]
+        _lib.FDs.argtypes = [dp, dp, dp, ctypes.c_int]
+        _lib.nullspace.argtypes = [dp, dp, ctypes.c_int, ctypes.POINTER(ctypes.c_int)]
+        _lib.nullspace.restype = ctypes.c_int
+        _lib.SuperFastHash.argtypes = [ctypes.c_char_p, ctypes.c_int]
+        _lib.SuperFastHash.restype = ctypes.c_uint32
+        _lib.nsamples.argtypes = [ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_double]
+        _lib.svduv.argtypes = [dp, dp, dp, ctypes.c_int, dp, ctypes.c_int]
+        _lib.ref_minv3.argtypes = [dp]
+        _lib.ref_minv3.restype = ctypes.c_int
         if hasattr(_lib, "ref_find_homography_2el"):
             _lib.ref_find_homography_2el.argtypes = [dp, ctypes.c_int, ctypes.c_double, ctypes.c_double, ctypes.c_int,
                                                      ctypes.c_int, ctypes.c_uint64, dp, ctypes.POINTER(ctypes.c_ubyte),
@@ -144,3 +154,66 @@ def h_from_2el(ua, ub):
     h = np.zeros(9)
     ok = lib().ref_h_from_2el(_dptr(ua), _dptr(ub), _dptr(h))
     return bool(ok), h
+
+
+# ---- single leaves of the reference, for known-answer tests of the engine's restatements of them
+def fds(u6, F):
+    """FDs (Ftools.c): Sampson residuals of F[9] on rows (x1, y1, 1, x2, y2, 1)."""
+    u = np.ascontiguousarray(u6, dtype=np.float64); F = np.ascontiguousarray(F, dtype=np.float64)
+    out = np.zeros(len(u))
+    lib().FDs(_dptr(u), _dptr(F), _dptr(out), len(u))
+    return out
+
+
+def nullspace(M):
+    """nullspace (utools.c) of a 9x9 matrix; returns (dimension, the 81 doubles it writes)."""
+    a = np.ascontiguousarray(M, dtype=np.float64).copy()
+    out = np.zeros(81)
+    buf = (ctypes.c_int * 18)()
+    k = lib().nullspace(_dptr(a), _dptr(out), 9, buf)
+    return k, out
+
+
+def superfasthash(idx):
+    """SuperFastHash (hash.c) of an int32 index list, as the reference hashes its samples."""
+    b = np.ascontiguousarray(idx, dtype=np.int32).tobytes()
+    return lib().SuperFastHash(b, len(b))
+
+
+def nsamples(ni, n, s, conf):
+    """nsamples (rtools.c): iterations needed for confidence conf with ni inliers of n, samples of size s."""
+    return lib().nsamples(ni, n, s, conf)
+
+
+def svd_v(A):
+    """svduv (CCMATH) of a 3x3 matrix: the right singular vectors as columns, in CCMATH's (unsorted) order."""
+    a = np.ascontiguousarray(A, dtype=np.float64).copy()
+    d = np.zeros(3); u = np.zeros(9); v = np.zeros(9)
+    lib().svduv(_dptr(d), _dptr(a), _dptr(u), 3, _dptr(v), 3)
+    return v.reshape(3, 3)
+
+
+def value31(seed, k, j):
+    """The harness' Philox stream: 31-bit value j of iteration k."""
+    return lib().ref_value31(seed, k, j)
+
+
+def stateless_sample(seed, k, N, m):
+    """The harness' stateless minimal sample of iteration k: m distinct indices of N."""
+    sel = (ctypes.c_int * 8)()
+    lib().ref_stateless_sample(ctypes.c_uint64(seed), k, N, m, sel)
+    return np.array(list(sel)[:m], dtype=np.int32)
+
+
+def row_digests(a):
+    """8-byte digest of each row of a [K, M] float64 array, NaNs canonicalised (all NaNs compare equal)."""
+    a = np.where(np.isnan(a), np.nan, a)
+    return np.array([int.from_bytes(hashlib.sha1(r.tobytes()).digest()[:8], "little") for r in a], dtype=np.uint64)
+
+
+def minv3_digests(mats):
+    """CCMATH minv (matutls/minv.c) on each row of mats [K, 9] taken as a 3x3 matrix, in place.  Returns the return
+    codes and the row_digests of the matrices it leaves: a bit-for-bit record small enough to store."""
+    out = np.ascontiguousarray(mats, dtype=np.float64).copy()
+    rc = np.array([lib().ref_minv3(_dptr(row)) for row in out], dtype=np.int32)
+    return rc, row_digests(out)

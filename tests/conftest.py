@@ -26,7 +26,11 @@ def norm_model(M):
 
 @pytest.fixture(scope="session")
 def ref_oracle():
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("oracle/_ref/libdegensac_ref.so not built (run oracle/build_ref.sh where /root/reference exists)")
-    return ref
+    """The original project's answers (tests/reference_calls.py): replayed from golden data, or answered by the compiled
+    reference and recorded to the file DGB200_RECORD_REFERENCE names."""
+    from tests.reference_calls import ReferenceCalls
+    record_to = os.environ.get("DGB200_RECORD_REFERENCE")
+    oracle = ReferenceCalls(record_to)
+    yield oracle
+    if record_to:
+        oracle.save()

@@ -2,6 +2,8 @@
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -46,21 +48,26 @@ def test_argument_errors_before_any_cuda_call():
 
 
 def test_no_cpu_fallback_without_gpu():
-    """Without a CUDA device every compute entry point must fail loudly."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+    """Without a CUDA device every compute entry point must fail loudly (checked in a child process that sees no
+    device, so that it runs on GPU machines too)."""
     if not os.path.exists(LIB):
         pytest.skip("libdegensac_b200.so not built")
-    import pydegensac_b200 as pdg
-    from pydegensac_b200.scenes import scene_F
-    p1, p2, _ = scene_F(50, 0.5, 0)
-    with pytest.raises(RuntimeError):
-        pdg.findFundamentalMatrix(p1, p2, 1.0, 0.99, 100, seed=1)
-    with pytest.raises(RuntimeError):
-        pdg.findHomography(p1, p2, 1.0, 0.99, 100, seed=1)
-    with pytest.raises(RuntimeError):
-        pdg.findFundamentalMatrixBatch(p1[None], p2[None], 1.0, 0.99, 100)
+    code = """if True:
+        import pytest, torch
+        assert not torch.cuda.is_available()
+        import pydegensac_b200 as pdg
+        from pydegensac_b200.scenes import scene_F
+        p1, p2, _ = scene_F(50, 0.5, 0)
+        with pytest.raises(RuntimeError):
+            pdg.findFundamentalMatrix(p1, p2, 1.0, 0.99, 100, seed=1)
+        with pytest.raises(RuntimeError):
+            pdg.findHomography(p1, p2, 1.0, 0.99, 100, seed=1)
+        with pytest.raises(RuntimeError):
+            pdg.findFundamentalMatrixBatch(p1[None], p2[None], 1.0, 0.99, 100)
+    """
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-3000:]
 
 
 def test_python_validation_matches_reference_layer():

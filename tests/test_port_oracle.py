@@ -1,5 +1,5 @@
-"""Pins the plain-C restatement (oracle/port) against the golden vectors produced by the unmodified reference and,
-when oracle/_ref is present, against the reference itself on randomised inputs."""
+"""Pins the plain-C restatement (oracle/port) against the golden vectors produced by the unmodified reference and
+against the reference's recorded answers on randomised inputs."""
 import json
 import os
 
