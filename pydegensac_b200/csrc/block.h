@@ -10,19 +10,14 @@
 
 namespace dg {
 
-constexpr int kMaxWarps = 16;      // group size <= 512 threads
+// The CTA has 8 warps.  red_d / red_i have 16 slots because blk_inlidxs_ballot<2> uses the two halves of red_i as
+// the warp counts of its two thresholds.
+constexpr int kMaxWarps = 16;
 constexpr int kVecRed = 48;        // widest vector reduction (45 covariance entries)
-// warps of one group as far as the scratch layout is concerned (both nvcc passes must agree on sizeof(BlockScratch);
-// the one-thread host emulation keeps the full layout)
-#if defined(__CUDACC__)
-constexpr int kGroupWarpsScratch = DG_GROUP_WARPS;
-#else
-constexpr int kGroupWarpsScratch = kMaxWarps;
-#endif
 // `vec` doubles as the row buffer of the one-warp small fits (hfit.h: 2 x 32 DLT rows of 9) and as the swap-partner
-// buffer of the plane-and-parallax waves, hence the floor of 576 doubles.
-constexpr int kVecDoubles = (kGroupWarpsScratch >= 8 ? kMaxWarps : kGroupWarpsScratch) * kVecRed > 576
-                                ? (kGroupWarpsScratch >= 8 ? kMaxWarps : kGroupWarpsScratch) * kVecRed : 576;
+// buffer of the plane-and-parallax waves, hence at least 576 doubles.
+constexpr int kVecDoubles = kMaxWarps * kVecRed;
+static_assert(kVecDoubles >= 576, "vec holds the small fits' rows and the plane-and-parallax swap partners");
 
 struct BlockScratch {
   double red_d[kMaxWarps];
@@ -37,7 +32,7 @@ struct BlockScratch {
   double fh_F[15 * 9];             // ... and the models
   WarpScratch ws[1];               // warp 0's tile for the cooperative 9x9 / 8x9 solves
   union {                          // never live at the same time:
-    WarpScratch wsx[kGroupWarpsScratch >= 5 ? 4 : 1];   //   tiles of warps 1..4 (the five checksample triplets run side by side)
+    WarpScratch wsx[4];            //   tiles of warps 1..4 (the five checksample triplets run side by side)
     double vec[kVecDoubles];       //   per-warp slots of the wide block reductions
   };
   DG_ENG WarpScratch* warp_tile(int wid) { return wid == 0 ? &ws[0] : &wsx[wid - 1]; }
@@ -175,23 +170,10 @@ DG_ENG inline void blk_scan_sum(const Ctx& c, int cnt, double J, int* off, int* 
 DG_ENG inline double ld_row(const double* p) { return __ldcg(p); }
 DG_ENG inline void st_row(double* p, double v) { __stcg(p, v); }
 DG_ENG inline void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
-// correspondences read by the streaming O(N) passes (every residual row reads all four SoA rows once): DG_SOA_LD = 1
-// keeps them from allocating in L1, 2 = L2 only (ld.cg; measured best: +5 %, the L1 lines the serial steps live on --
-// stack, lists, hypothesis queue -- are no longer swept out by every residual row), 0 = default caching
-#ifndef DG_SOA_LD
-#define DG_SOA_LD 2
-#endif
-DG_ENG inline double ld_soa(const double* p) {
-#if DG_SOA_LD == 1
-  double v;
-  asm("ld.global.L1::no_allocate.f64 %0, [%1];" : "=d"(v) : "l"(p));
-  return v;
-#elif DG_SOA_LD == 2
-  return __ldcg(p);
-#else
-  return *p;
-#endif
-}
+// correspondences read by the streaming O(N) passes (every residual row reads all four SoA rows once): L2 only
+// (ld.cg; measured +5 % over default caching: the L1 lines the serial steps live on -- stack, lists, hypothesis
+// queue -- are no longer swept out by every residual row)
+DG_ENG inline double ld_soa(const double* p) { return __ldcg(p); }
 #else
 inline double ld_row(const double* p) { return *p; }
 inline void st_row(double* p, double v) { *p = v; }
@@ -206,7 +188,7 @@ inline double ld_soa(const double* p) { return *p; }
 // chunk [w*chunk, (w+1)*chunk) of the row (chunk a multiple of 32); its lanes stride the chunk 32 residuals at a time,
 // so the loads are coalesced and the ballot of "e <= th" IS the order.  The ballot word of trip j is parked on lane j
 // (chunks up to 1024 residuals), the warp totals are scanned across the CTA, then the parked words are replayed to
-// write the indices -- the row is read once (the thread-segment fallback below reads it twice, uncoalesced).
+// write the indices -- the row is read once (the host emulation's thread-segment loop below reads it twice).
 // NTH = 1: (S[0], lists[0]) for th[0];  NTH = 2: both thresholds from the same pass.
 template <int NTH>
 __device__ __noinline__ void blk_inlidxs_ballot(const Ctx& c, const double* __restrict__ err, const double* th,
@@ -221,29 +203,6 @@ __device__ __noinline__ void blk_inlidxs_ballot(const Ctx& c, const double* __re
     wq[t] = th[t] * 9 / 4;
     winv[t] = (th[t] == 0) ? 0.0 : 1.0 / wq[t];
     J[t] = 0.0; off[t] = 0; cnt[t] = 0; parked[t] = 0u;
-  }
-  if (c.nw == 1) {   // one warp owns the row: single pass, running offsets
-    #pragma unroll 1
-    for (int base = 0; base < c.N; base += 64) {
-      const int i0 = base + c.lane, i1 = i0 + 32;
-      const double e0 = (i0 < c.N) ? ld_row(err + i0) : INFINITY;
-      const double e1 = (i1 < c.N) ? ld_row(err + i1) : INFINITY;
-#pragma unroll
-      for (int t = 0; t < NTH; ++t) {
-        if (th[t] != 0 && !(e0 >= wq[t])) J[t] += 1 - e0 * winv[t];
-        if (th[t] != 0 && !(e1 >= wq[t])) J[t] += 1 - e1 * winv[t];
-        const bool in0 = e0 <= th[t], in1 = e1 <= th[t];
-        const unsigned m0 = __ballot_sync(full, in0), m1 = __ballot_sync(full, in1);
-        const int o1 = off[t] + __popc(m0);
-        if (in0) lists[t][off[t] + __popc(m0 & lt)] = i0;
-        if (in1) lists[t][o1 + __popc(m1 & lt)] = i1;
-        off[t] = o1 + __popc(m1);
-      }
-    }
-#pragma unroll
-    for (int t = 0; t < NTH; ++t) { S[t] = make_score(); S[t].J = warp_sum(J[t]); S[t].I = (unsigned)off[t]; }
-    __syncwarp();
-    return;
   }
   const int chunk = (((c.N + c.nw - 1) / c.nw) + 31) & ~31;
   const int wbeg = c.wid * chunk;
@@ -343,15 +302,13 @@ DG_ENGN Score blk_inlidxs(const Ctx& c, const double* err, double th, int* list)
       if (e[j] <= th) list[off++] = beg + j;
   } else {
 #if DG_DEVICE_PASS
-    if (c.nw <= kMaxWarps / 2) {
-      const double tha[1] = {th};
-      int* const la[1] = {list};
-      Score Sa[1];
-      blk_inlidxs_ballot<1>(c, err, tha, la, Sa);
-      DG_PROF_END(21);
-      return Sa[0];
-    }
-#endif
+    const double tha[1] = {th};
+    int* const la[1] = {list};
+    Score Sa[1];
+    blk_inlidxs_ballot<1>(c, err, tha, la, Sa);
+    DG_PROF_END(21);
+    return Sa[0];
+#else
     #pragma unroll 1
     for (int i = beg; i < end; ++i) {
       const double e = ld_row(err + i);
@@ -362,6 +319,7 @@ DG_ENGN Score blk_inlidxs(const Ctx& c, const double* err, double th, int* list)
     #pragma unroll 1
     for (int i = beg; i < end; ++i)
       if (ld_row(err + i) <= th) list[off++] = i;
+#endif
   }
   s.J = Jtot;
   s.I = (unsigned)total;
@@ -379,17 +337,15 @@ DG_ENGN void blk_inlidxs2(const Ctx& c, const double* err, double thA, int* list
   const int per = (c.N + c.nt - 1) / c.nt;
   if (per > 8 || c.N >= 65536) {
 #if DG_DEVICE_PASS
-    if (c.nw <= kMaxWarps / 2) {
-      const double tha[2] = {thA, thB};
-      int* const la[2] = {listA, listB};
-      Score Sa[2];
-      blk_inlidxs_ballot<2>(c, err, tha, la, Sa);
-      *SA = Sa[0]; *SB = Sa[1];
-      return;
-    }
-#endif
+    const double tha[2] = {thA, thB};
+    int* const la[2] = {listA, listB};
+    Score Sa[2];
+    blk_inlidxs_ballot<2>(c, err, tha, la, Sa);
+    *SA = Sa[0]; *SB = Sa[1];
+#else
     *SA = blk_inlidxs(c, err, thA, listA);
     *SB = blk_inlidxs(c, err, thB, listB);
+#endif
     return;
   }
   DG_PROF_BEGIN(21);

@@ -23,25 +23,10 @@
 #define DG_ENGN inline
 #endif
 
-// A pair is owned by a GROUP of DG_GROUP_WARPS warps: all DG_CTA_WARPS warps of the CTA (the default, cooperative
-// design) or fewer (1, 2, 4: a CTA then hosts DG_CTA_WARPS / DG_GROUP_WARPS pairs side by side; build-time experiment,
-// DESIGN.md section 7).  Groups never synchronise with each other: DG_SYNC() is the CTA barrier, a named barrier
-// (bar.sync 1+group, 32*G) or __syncwarp.  The engine code only sees its group through Ctx {tid, nt, wid, nw}.
-#ifndef DG_CTA_WARPS
-#define DG_CTA_WARPS 8
-#endif
-#ifndef DG_GROUP_WARPS
-#define DG_GROUP_WARPS DG_CTA_WARPS
-#endif
+// One CTA owns one pair: DG_SYNC() is the CTA barrier (a no-op in the one-thread host emulation).
 #if defined(__CUDA_ARCH__)
 #define DG_DEVICE_PASS 1
-#if DG_GROUP_WARPS == 1
-#define DG_SYNC() __syncwarp()
-#elif DG_GROUP_WARPS == DG_CTA_WARPS
 #define DG_SYNC() __syncthreads()
-#else
-#define DG_SYNC() asm volatile("bar.sync %0, %1;" ::"r"(1 + (int)(threadIdx.x / (32 * DG_GROUP_WARPS))), "n"(32 * DG_GROUP_WARPS) : "memory")
-#endif
 #else
 #define DG_DEVICE_PASS 0
 #define DG_SYNC() ((void)0)
@@ -50,7 +35,7 @@
 // Optional phase profiling (build with -DDG_PROF): thread 0 of every CTA accumulates clock64() deltas.
 #if defined(DG_PROF) && DG_DEVICE_PASS
 extern __device__ unsigned long long g_dg_prof[64];
-#define DG_PROF_LEAD() ((threadIdx.x % (32 * DG_GROUP_WARPS)) == 0)
+#define DG_PROF_LEAD() (threadIdx.x == 0)
 #define DG_PROF_BEGIN(id) long long prof_t_##id = DG_PROF_LEAD() ? clock64() : 0
 #define DG_PROF_END(id) do { if (DG_PROF_LEAD()) atomicAdd(&g_dg_prof[id], (unsigned long long)(clock64() - prof_t_##id)); } while (0)
 #define DG_PROF_COUNT(id, n) do { if (DG_PROF_LEAD()) atomicAdd(&g_dg_prof[id], (unsigned long long)(n)); } while (0)

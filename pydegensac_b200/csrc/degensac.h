@@ -430,7 +430,7 @@ DG_ENGN void blk_inner_FH(const Ctx& c, Workspace& W, const int* uH, int nH, con
   {
     double* fhF = c.sc->fh_F;
     int* fhC = c.sc->fh_cnt;
-    const int nfit = (kGroupWarpsScratch >= 5 && c.nw >= 5) ? 5 : 1;   // warp tiles available side by side
+    const int nfit = (c.nw >= 5) ? 5 : 1;   // warp tiles available side by side
     #pragma unroll 1
     for (int base = 0; base < 15; base += nfit) {
       DG_SYNC();

@@ -4,7 +4,7 @@
 // work counter:
 //   * the pair's correspondences are read ONCE from HBM (coalesced 16-byte loads of the [n][dim] rows) and
 //     de-interleaved into a structure-of-arrays copy (4 x n doubles) in the CTA's slab of global memory -- L1/L2
-//     resident; shared-memory residency measured slower, see the launch plan below -- plus the centred FP32 tile of the
+//     resident; shared-memory residency measured slower, see the CTA shape below -- plus the centred FP32 tile of the
 //     wave filter (pair-interleaved, 16 B per correspondence);
 //   * engine_f.h / engine_h.h run the speculative hypothesis WAVES (two threads per 7-point sample / one per 4-point
 //     sample, one warp per scored model, FP32 upper-bound filter with packed FFMA2) and the ordered REPLAY (LO, DEGENSAC,
@@ -34,65 +34,41 @@ __device__ unsigned long long g_dg_prof[64];
 
 namespace {
 
-#ifndef DG_LB_THREADS
-#define DG_LB_THREADS 256
-#endif
-#ifndef DG_LB_BLOCKS
-#define DG_LB_BLOCKS 2
-#endif
-constexpr int kMaxThreads = DG_LB_THREADS;
-constexpr int kChunkDefault = 512;
-int cfg_chunk() {   // iterations hypothesised per wave (DGB200_CHUNK, multiple of 128)
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DGB200_CHUNK"); v = e ? atoi(e) : kChunkDefault; if (v < 128) v = 128; if (v > 4096) v = 4096; v = (v / 128) * 128; }
-  return v;
-}
-#define kChunk cfg_chunk()
-
-// CTA shape.  256 threads x 2 CTAs per SM measured fastest on B200 (profiles/README.md): the waves and the O(N)
-// passes of the replay want the 8 warps, while more, smaller CTAs per SM lose to instruction-cache misses (each
-// CTA walks a different part of a ~300 KB code image).  FP64 correspondences live in the per-CTA global slab
-// (L1/L2 resident), the FP32 filter tile in shared memory.  DGB200_THREADS / DGB200_SMEM_TILE override for experiments.
-int cfg_threads() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("DGB200_THREADS");
-    v = e ? atoi(e) : 256;
-    if (v < 32) v = 32;
-    if (v > kMaxThreads) v = kMaxThreads;
-    v = (v / 32) * 32;
-  }
-  return v;
-}
-int cfg_smem_tile() {
-  static int v = -2;
-  if (v < -1) { const char* e = getenv("DGB200_SMEM_TILE"); v = e ? atoi(e) : 0; }   // measured on B200: the L1 capacity the tile takes away costs more than it saves
-  return v;
-}
+// CTA shape.  256 threads x 2 CTAs per SM measured fastest on B200 (DESIGN.md sections 3.1 and 7): the waves and the
+// O(N) passes of the replay want the 8 warps, while more, smaller CTAs per SM lose to instruction-cache misses (each
+// CTA walks a different part of a ~300 KB code image).  Shared memory holds the block scratch only; the pair's FP64
+// correspondences and FP32 filter tile live in the CTA's slab (L1/L2 resident), which measured faster than shared
+// memory because the serial steps need that L1 capacity.
+constexpr int kThreads = 256;
+constexpr int kCtasPerSm = 2;
+constexpr int kChunk = 512;   // iterations hypothesised per wave
 
 int env_int(const char* name, int dflt) {
   const char* e = getenv(name);
   return e ? atoi(e) : dflt;
 }
 
-struct BatchArgs {
-  const double* x1y1;
-  const double* x2y2;
-  const int* offsets;   // ragged batches: pair p owns rows offsets[p] .. offsets[p+1] of the concatenated arrays; nullptr: n each
-  int n_pairs, n, dim;  // n: correspondences per pair (ragged: the largest, which sizes the slabs)
-  double px_th, conf, laf_coef;
-  int max_iters, metric, sym_check, degen;
-  unsigned flags;       // DGB200_FLAG_*
-  const unsigned long long* seeds;
-  double* model_out;
-  unsigned char* mask_out;
-  int* stats_out;
+// One batch as the caller passed it; the fields an entry point does not take keep these zeros.
+struct Job {
+  const double* x1y1 = nullptr;
+  const double* x2y2 = nullptr;
+  const int32_t* offsets = nullptr;   // ragged batches: pair p owns rows offsets[p] .. offsets[p+1] of the concatenated arrays; nullptr: n each
+  int n_pairs = 0, n = 0, dim = 0;    // n: correspondences per pair (ragged: the largest, which sizes the slabs)
+  double px_th = 0, conf = 0, laf_coef = 0;
+  int max_iters = 0, metric = 0, sym_check = 0, degen = 0;
+  unsigned flags = 0;                 // DGB200_FLAG_*
+  const uint64_t* seeds = nullptr;
+  double* model_out = nullptr;
+  uint8_t* mask_out = nullptr;
+  int32_t* stats_out = nullptr;
+};
+
+// A Job on the device plus what launch() derives for the kernel.
+struct BatchArgs : Job {
   unsigned char* workspace;
   size_t ws_stride;
   int chunk;
   int* work_counter;
-  int pts_in_smem;
-  int tile32_in_smem;   // FP32 filter tile placement (F path)
   int aligned16;        // both input pointers 16-byte aligned: dim == 2 rows are read as double2
   int filter32;         // FP32 upper-bound filter in the F wave (DGB200_FILTER32=0 scores the wave in FP64; same results)
   const int* ready;     // host-buffer flavour: number of leading pairs whose input has landed in HBM (nullptr: all)
@@ -101,32 +77,21 @@ struct BatchArgs {
 };
 
 template <int KIND>  // 0: fundamental matrix, 1: homography, 2: homography from elliptical features (rows u10, engine_h2el.h)
-__global__ void __launch_bounds__(kMaxThreads, DG_LB_BLOCKS) ransac_pairs_kernel(BatchArgs a) {
+__global__ void __launch_bounds__(kThreads, kCtasPerSm) ransac_pairs_kernel(BatchArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  // The CTA hosts blockDim.x / GT groups (one in the default build); each owns one pair at a time, its own scratch,
-  // slab and barrier.
-  constexpr int GT = (DG_GROUP_WARPS == DG_CTA_WARPS) ? 0 : 32 * DG_GROUP_WARPS;   // 0: the group is the whole CTA
-  const int gthreads = GT ? GT : (int)blockDim.x;
-  const int gid = GT ? (int)threadIdx.x / GT : 0, ngroups = GT ? (int)blockDim.x / GT : 1;
-  const int gtid = GT ? (int)threadIdx.x % GT : (int)threadIdx.x;
-  const size_t sc_bytes = dg::align_up(sizeof(dg::BlockScratch), 128);
-  dg::BlockScratch* sc = reinterpret_cast<dg::BlockScratch*>(smem_raw + (size_t)gid * sc_bytes);
-  unsigned char* slab = a.workspace + ((size_t)blockIdx.x * ngroups + gid) * a.ws_stride;
+  const int tid = (int)threadIdx.x, nt = (int)blockDim.x;
+  dg::BlockScratch* sc = reinterpret_cast<dg::BlockScratch*>(smem_raw);
+  unsigned char* slab = a.workspace + (size_t)blockIdx.x * a.ws_stride;
   dg::Workspace W;
-  double* soa_global;
+  double* soa;
   const bool use_laf = (a.laf_coef > 0) && (a.dim == 6);
-  dg::workspace_carve(slab, a.n, a.chunk, use_laf, &W, &soa_global);
+  dg::workspace_carve(slab, a.n, a.chunk, use_laf, &W, &soa);
   const size_t row = dg::align_up(sizeof(double) * (size_t)a.n, 128) / sizeof(double);
-  double* soa = a.pts_in_smem ? reinterpret_cast<double*>(smem_raw + sc_bytes) : soa_global;
-  const size_t soa_smem_bytes = a.pts_in_smem ? dg::align_up(sizeof(double) * (size_t)a.n, 128) * 4 : 0;
-  dg::Pt32* tile32 = a.tile32_in_smem
-                         ? reinterpret_cast<dg::Pt32*>(smem_raw + (size_t)ngroups * sc_bytes + soa_smem_bytes +
-                                                       (size_t)gid * dg::align_up(16 * ((size_t)a.n + 1), 128))
-                         : reinterpret_cast<dg::Pt32*>(dg::workspace_tile32(slab, a.n, a.chunk, use_laf));
+  dg::Pt32* tile32 = reinterpret_cast<dg::Pt32*>(dg::workspace_tile32(slab, a.n, a.chunk, use_laf));
   dg::Tile32 t32;
 
   dg::Ctx c;
-  c.tid = gtid; c.nt = gthreads; c.lane = gtid & 31; c.wid = gtid >> 5; c.nw = gthreads >> 5;
+  c.tid = tid; c.nt = nt; c.lane = tid & 31; c.wid = tid >> 5; c.nw = nt >> 5;
   c.N = a.n;
   c.x1 = soa; c.y1 = soa + row; c.x2 = soa + 2 * row; c.y2 = soa + 3 * row;
   c.sc = sc;
@@ -135,7 +100,7 @@ __global__ void __launch_bounds__(kMaxThreads, DG_LB_BLOCKS) ransac_pairs_kernel
 
   for (;;) {
     DG_SYNC();
-    if (gtid == 0) sc->pair = atomicAdd(a.work_counter, 1);
+    if (tid == 0) sc->pair = atomicAdd(a.work_counter, 1);
     DG_SYNC();
     const int p = sc->pair;
     if (p >= a.n_pairs) break;
@@ -144,7 +109,7 @@ __global__ void __launch_bounds__(kMaxThreads, DG_LB_BLOCKS) ransac_pairs_kernel
       // chunk.  The wait is bounded: when copies cannot overlap the kernel (a profiler serialising the streams, a
       // stalled link) the CTA records the pair, raises the abort flag and retires; the host then runs the pairs from
       // the smallest recorded index on in a second, ordinary launch.  Nothing can hang.
-      if (gtid == 0) {
+      if (tid == 0) {
         int ok = (*reinterpret_cast<volatile int*>(a.status) == 0) ? 1 : 0;
         if (ok) {
           const long long t0 = clock64();
@@ -168,12 +133,12 @@ __global__ void __launch_bounds__(kMaxThreads, DG_LB_BLOCKS) ransac_pairs_kernel
     if (a.dim == 2 && a.aligned16) {   // rows are 16 bytes, so every pair of a ragged batch starts aligned too
       const double2* v1 = reinterpret_cast<const double2*>(g1);
       const double2* v2 = reinterpret_cast<const double2*>(g2);
-      for (int i = gtid; i < n; i += gthreads) {
+      for (int i = tid; i < n; i += nt) {
         const double2 q1 = __ldcg(v1 + i), q2 = __ldcg(v2 + i);   // L2 only: the chunk may have landed after this kernel started
         soa[i] = q1.x; soa[row + i] = q1.y; soa[2 * row + i] = q2.x; soa[3 * row + i] = q2.y;
       }
     } else {
-      for (int i = gtid; i < n; i += gthreads) {
+      for (int i = tid; i < n; i += nt) {
         const double* q1 = g1 + (size_t)i * a.dim;
         const double* q2 = g2 + (size_t)i * a.dim;
         soa[i] = __ldcg(q1); soa[row + i] = __ldcg(q1 + 1);
@@ -188,7 +153,6 @@ __global__ void __launch_bounds__(kMaxThreads, DG_LB_BLOCKS) ransac_pairs_kernel
     const unsigned long long seed = a.seeds ? a.seeds[p] : (unsigned long long)p;
     double* model = a.model_out + (size_t)p * 9;
     unsigned char* mask = a.mask_out + row0;
-    int local_stats[4];
     int* s_stats = sc->stats;
     if (KIND == 0) {
       c.t32 = nullptr;
@@ -227,9 +191,8 @@ __global__ void __launch_bounds__(kMaxThreads, DG_LB_BLOCKS) ransac_pairs_kernel
     double asum = 0.0;
     for (int i = 0; i < 9; ++i) asum += fabs(model[i]);
     if (asum == 0.0)
-      for (int i = gtid; i < n; i += gthreads) mask[i] = 0;
-    if (a.stats_out && gtid < 4) a.stats_out[(size_t)p * 4 + gtid] = s_stats[gtid];
-    (void)local_stats;
+      for (int i = tid; i < n; i += nt) mask[i] = 0;
+    if (a.stats_out && tid < 4) a.stats_out[(size_t)p * 4 + tid] = s_stats[tid];
   }
 }
 
@@ -247,7 +210,6 @@ struct LaunchCtx {
 struct Cache {
   int device = -1;
   int sm_count = 0;
-  size_t smem_optin = 0;
   std::vector<LaunchCtx> ctxs;
   unsigned char* io = nullptr; size_t io_bytes = 0;   // staging for the host-buffer flavour
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev_feed = nullptr;
@@ -302,7 +264,6 @@ int ensure_device() {
   CU(cudaGetDeviceProperties(&prop, dev));
   Cache c;
   c.sm_count = prop.multiProcessorCount;
-  c.smem_optin = prop.sharedMemPerBlockOptin;
   cudaError_t err = cudaSuccess;
   auto step = [&](cudaError_t r) { if (err == cudaSuccess) err = r; };
   step(cudaEventCreate(&c.ev0));
@@ -351,70 +312,24 @@ int acquire_ctx(cudaStream_t st, size_t need, LaunchCtx** out) {
   return 0;
 }
 
-struct Job {
-  const double* d1; const double* d2; const int* d_offsets;
-  int n_pairs, n, dim;
-  double px_th, conf, laf_coef;
-  int max_iters, metric, sym_check, degen;
-  unsigned flags;
-  const unsigned long long* d_seeds;
-  double* d_model; unsigned char* d_mask; int* d_stats;
-};
-
 template <int KIND>
-int launch(const Job& j, cudaStream_t st, const int* d_ready = nullptr, int* d_status = nullptr, long long wait_cycles = 0) {
+int launch(const Job& j, cudaStream_t st, const int* ready = nullptr, int* status = nullptr, long long wait_cycles = 0) {
   BatchArgs a;
-  a.ready = d_ready; a.status = d_status; a.wait_cycles = wait_cycles;
-  a.x1y1 = j.d1; a.x2y2 = j.d2; a.offsets = j.d_offsets; a.n_pairs = j.n_pairs; a.n = j.n; a.dim = j.dim;
-  a.px_th = j.px_th; a.conf = j.conf; a.laf_coef = j.laf_coef; a.max_iters = j.max_iters; a.metric = j.metric;
-  a.sym_check = j.sym_check; a.degen = j.degen; a.flags = j.flags; a.seeds = j.d_seeds;
-  a.model_out = j.d_model; a.mask_out = j.d_mask; a.stats_out = j.d_stats;
+  static_cast<Job&>(a) = j;
+  a.ready = ready; a.status = status; a.wait_cycles = wait_cycles;
   a.chunk = kChunk;
-  const int n = j.n;
-  constexpr int kGroups = DG_CTA_WARPS / DG_GROUP_WARPS;                      // pairs side by side per CTA (1 by default)
-  const size_t sc_bytes = dg::align_up(sizeof(dg::BlockScratch), 128) * kGroups;
-  const size_t tile = dg::align_up(sizeof(double) * (size_t)n, 128) * 4;       // FP64 SoA of the pair
-  const size_t tile32 = (16 * ((size_t)n + 1) <= 98304) ? dg::align_up(16 * ((size_t)n + 1), 128) * kGroups : 0;   // FP32 filter tile(s) (pair-interleaved: N+1 slots)
-  const int kThreads = (kGroups > 1) ? 32 * DG_CTA_WARPS : cfg_threads();
-  auto kern = ransac_pairs_kernel<KIND>;
-  // Shared-memory plan: block scratch always; the FP32 filter tile when it fits.  The FP64 correspondences stay in
-  // global memory (L1/L2-resident): DGB200_SMEM_TILE=1 moves them to shared memory too, which measured 12 % slower
-  // at N = 2000 (10.2k vs 11.6k pairs/s) because the residual rows and lists then lose their L1 capacity.
-  size_t smem = sc_bytes;
-  a.pts_in_smem = 0;
-  a.tile32_in_smem = 0;
   a.filter32 = (env_int("DGB200_FILTER32", 1) != 0 && (KIND == 0 || (KIND == 1 && j.metric == dg::H_SAMPSON))) ? 1 : 0;   // parity switch, read at every launch
-  a.aligned16 = ((((uintptr_t)j.d1) | ((uintptr_t)j.d2)) & 15) == 0 ? 1 : 0;
-  if (tile32 && a.filter32 && smem + tile32 <= g_c.smem_optin && env_int("DGB200_TILE32_SMEM", 0) != 0) {
-    // DGB200_TILE32_SMEM=1: the tile in shared memory (when DG_LB_BLOCKS CTAs per SM still fit).  Default: in the slab,
-    // served by L1 -- measured 1.4 % faster at N = 2000 (16.37k vs 16.15k pairs/s): the 64 KB of L1 per SM the two
-    // tiles would take are worth more to the serial steps (stack, lists, queue) than shared-memory residency to the wave
-    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem + tile32)));
-    int occ = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kThreads, smem + tile32));
-    if (occ >= DG_LB_BLOCKS) { a.tile32_in_smem = 1; smem += tile32; }
-  }
+  a.aligned16 = ((((uintptr_t)j.x1y1) | ((uintptr_t)j.x2y2)) & 15) == 0 ? 1 : 0;
+  const size_t smem = dg::align_up(sizeof(dg::BlockScratch), 128);
+  auto kern = ransac_pairs_kernel<KIND>;
   int per_sm = 0;
-  const int want_tile = cfg_smem_tile();
-  if (want_tile != 0 && kGroups == 1 && smem + tile <= g_c.smem_optin) {
-    const size_t smem_full = smem + tile;
-    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_full));
-    int occ = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kThreads, smem_full));
-    if (occ >= 2 || (want_tile > 0 && occ >= 1)) { a.pts_in_smem = 1; smem = smem_full; per_sm = occ; }
-  }
-  if (!a.pts_in_smem) {
-    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, smem));
-  }
+  CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kThreads, smem));
   if (per_sm < 1) return fail(DGB200_E_CUDA, "kernel does not fit on an SM");
-  { const int cap = env_int("DGB200_CTAS_PER_SM", 0); if (cap >= 1 && cap < per_sm) per_sm = cap; }
   int grid = g_c.sm_count * per_sm;     // persistent CTAs: a whole number of CTAs per SM
-  if ((long long)grid * kGroups > j.n_pairs) grid = (j.n_pairs + kGroups - 1) / kGroups;
-  a.ws_stride = dg::align_up(dg::workspace_bytes(n, a.chunk, j.laf_coef > 0 && j.dim == 6), 256);
-  const size_t need = a.ws_stride * (size_t)grid * kGroups;
+  if (grid > j.n_pairs) grid = j.n_pairs;
+  a.ws_stride = dg::align_up(dg::workspace_bytes(j.n, a.chunk, j.laf_coef > 0 && j.dim == 6), 256);
   LaunchCtx* lc = nullptr;
-  const int rc = acquire_ctx(st, need, &lc);
+  const int rc = acquire_ctx(st, a.ws_stride * (size_t)grid, &lc);
   if (rc) return rc;
   a.workspace = lc->ws;
   a.work_counter = lc->counter;
@@ -461,17 +376,18 @@ int check_offsets(int kind, const int32_t* offsets, int n_pairs, int* n_max, lon
 }
 
 template <int KIND>
-int run_host(const double* x1y1, const double* x2y2, const int32_t* offsets, int n_pairs, int n, int dim, double px_th,
-             double conf, int max_iters, int metric, int sym_check, double laf_coef, int degen, const uint64_t* seeds,
-             double* model_out, uint8_t* mask_out, int32_t* stats_out, unsigned flags = 0) {
+int run_host(const Job& h) {   // h: a batch in host memory
   std::lock_guard<std::mutex> lk(g_mu);
+  const int32_t* offsets = h.offsets;
+  const int n_pairs = h.n_pairs, dim = h.dim;
+  int n = h.n;
   long long rows = (long long)n_pairs * n;
   if (offsets) {
     if (n_pairs < 1) return fail(DGB200_E_ARG, "n_pairs must be >= 1");
     const int rc0 = check_offsets(KIND, offsets, n_pairs, &n, &rows);
     if (rc0) return rc0;
   }
-  int rc = check_args(KIND, x1y1, x2y2, n_pairs, n, dim, metric, laf_coef, model_out, mask_out);
+  int rc = check_args(KIND, h.x1y1, h.x2y2, n_pairs, n, dim, h.metric, h.laf_coef, h.model_out, h.mask_out);
   if (rc) return rc;
   rc = ensure_device();
   if (rc) return rc;
@@ -491,22 +407,20 @@ int run_host(const double* x1y1, const double* x2y2, const int32_t* offsets, int
   unsigned char* p = g_c.io;
   double* d1 = (double*)p; p += in_b;
   double* d2 = (double*)p; p += in_b;
-  unsigned long long* dseed = (unsigned long long*)p; p += seed_b;
-  int* doff = (int*)p; p += off_b;
+  uint64_t* dseed = (uint64_t*)p; p += seed_b;
+  int32_t* doff = (int32_t*)p; p += off_b;
   double* dmodel = (double*)p; p += model_b;
   unsigned char* dmask = p; p += mask_b;
   int* dstats = (int*)p;
-  Job j;
-  j.d1 = d1; j.d2 = d2; j.d_offsets = offsets ? doff : nullptr; j.n_pairs = n_pairs; j.n = n; j.dim = dim;
-  j.px_th = px_th; j.conf = conf; j.laf_coef = laf_coef; j.max_iters = max_iters; j.metric = metric;
-  j.sym_check = sym_check; j.degen = degen; j.flags = flags; j.d_seeds = seeds ? dseed : nullptr;
-  j.d_model = dmodel; j.d_mask = dmask; j.d_stats = dstats;
+  Job j = h;   // the same batch in the staging buffer
+  j.x1y1 = d1; j.x2y2 = d2; j.offsets = offsets ? doff : nullptr; j.n = n; j.seeds = h.seeds ? dseed : nullptr;
+  j.model_out = dmodel; j.mask_out = dmask; j.stats_out = dstats;
   // Input feed overlapped with the kernel: the batch is copied in chunks on a copy stream; after every chunk the
   // device-side `ready` count is bumped (a 4-byte copy from pinned memory, ordered behind the chunk) and the
   // persistent CTAs wait on it before staging a pair.  Chunk 0 covers the pairs the CTAs start with.
   cudaStream_t st = g_c.s_run, cs = g_c.s_copy;
   int nchunks = 8;
-  int first = 2 * DG_LB_BLOCKS * g_c.sm_count * (DG_CTA_WARPS / DG_GROUP_WARPS);   // two pairs per resident group
+  int first = 2 * kCtasPerSm * g_c.sm_count;   // two pairs per resident CTA
   if (first > n_pairs) first = n_pairs;
   int rest = n_pairs - first;
   if (rest <= 0) nchunks = 1;
@@ -517,7 +431,7 @@ int run_host(const double* x1y1, const double* x2y2, const int32_t* offsets, int
   const double feed_s = 2.0 * sizeof(double) * (double)rows * (double)dim / 4e9 + 0.020;
   long long wait_cycles = (long long)(feed_s * 2.1e9);
   if (const char* e = getenv("DGB200_FEED_WAIT_US")) wait_cycles = (long long)(atof(e) * 2.1e3);   // tests: force the fallback
-  if (seeds) CU(cudaMemcpyAsync(dseed, seeds, sizeof(uint64_t) * (size_t)n_pairs, cudaMemcpyHostToDevice, cs));
+  if (h.seeds) CU(cudaMemcpyAsync(dseed, h.seeds, sizeof(uint64_t) * (size_t)n_pairs, cudaMemcpyHostToDevice, cs));
   if (offsets) CU(cudaMemcpyAsync(doff, offsets, sizeof(int32_t) * ((size_t)n_pairs + 1), cudaMemcpyHostToDevice, cs));
   CU(cudaEventRecord(g_c.ev_feed, cs));
   CU(cudaStreamWaitEvent(st, g_c.ev_feed, 0));
@@ -532,9 +446,9 @@ int run_host(const double* x1y1, const double* x2y2, const int32_t* offsets, int
     if (done + cnt > n_pairs) cnt = n_pairs - done;
     const size_t off = row_of(done) * dim;
     const size_t elems = (row_of(done + cnt) - row_of(done)) * dim;
-    const cudaError_t e1 = cudaMemcpyAsync(d1 + off, x1y1 + off, sizeof(double) * elems, cudaMemcpyHostToDevice, cs);
+    const cudaError_t e1 = cudaMemcpyAsync(d1 + off, h.x1y1 + off, sizeof(double) * elems, cudaMemcpyHostToDevice, cs);
     const cudaError_t e2 = (KIND == 2) ? cudaSuccess   // one array of u10 rows
-                                       : cudaMemcpyAsync(d2 + off, x2y2 + off, sizeof(double) * elems, cudaMemcpyHostToDevice, cs);
+                                       : cudaMemcpyAsync(d2 + off, h.x2y2 + off, sizeof(double) * elems, cudaMemcpyHostToDevice, cs);
     done += cnt;
     g_c.h_ready[ci] = (e1 == cudaSuccess && e2 == cudaSuccess) ? done : n_pairs + 1;   // on a failed copy release the CTAs anyway
     cudaMemcpyAsync(g_c.ready, &g_c.h_ready[ci], sizeof(int), cudaMemcpyHostToDevice, cs);
@@ -556,9 +470,9 @@ int run_host(const double* x1y1, const double* x2y2, const int32_t* offsets, int
     if (from < n_pairs) {
       Job r = j;
       r.n_pairs = n_pairs - from;
-      r.d_seeds = seeds ? dseed + from : nullptr;
-      r.d_model = dmodel + (size_t)9 * from;
-      r.d_stats = dstats + (size_t)4 * from;
+      r.seeds = h.seeds ? dseed + from : nullptr;
+      r.model_out = dmodel + (size_t)9 * from;
+      r.stats_out = dstats + (size_t)4 * from;
       if (offsets) {
         // ragged: re-base the offsets of the remaining pairs (host copy, tiny)
         std::vector<int32_t> rebased((size_t)r.n_pairs + 1);
@@ -567,15 +481,15 @@ int run_host(const double* x1y1, const double* x2y2, const int32_t* offsets, int
         CU(cudaStreamSynchronize(st));
       }
       const size_t off = row_of(from);
-      r.d1 = d1 + off * dim; r.d2 = d2 + off * dim; r.d_mask = dmask + off;
+      r.x1y1 = d1 + off * dim; r.x2y2 = d2 + off * dim; r.mask_out = dmask + off;
       rc = launch<KIND>(r, st);
       if (rc) return rc;
       CU(cudaEventRecord(g_c.ev1, st));
     }
   }
-  CU(cudaMemcpyAsync(model_out, dmodel, sizeof(double) * 9 * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(mask_out, dmask, (size_t)rows, cudaMemcpyDeviceToHost, st));
-  if (stats_out) CU(cudaMemcpyAsync(stats_out, dstats, sizeof(int) * 4 * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(h.model_out, dmodel, sizeof(double) * 9 * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(h.mask_out, dmask, (size_t)rows, cudaMemcpyDeviceToHost, st));
+  if (h.stats_out) CU(cudaMemcpyAsync(h.stats_out, dstats, sizeof(int) * 4 * (size_t)n_pairs, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   float ms = 0.f;
   CU(cudaEventElapsedTime(&ms, g_c.ev0, g_c.ev1));
@@ -584,19 +498,12 @@ int run_host(const double* x1y1, const double* x2y2, const int32_t* offsets, int
 }
 
 template <int KIND>
-int run_dev(const double* d1, const double* d2, const int32_t* d_offsets, int n_pairs, int n, int dim, double px_th,
-            double conf, int max_iters, int metric, int sym_check, double laf_coef, int degen, const uint64_t* d_seeds,
-            double* d_model, uint8_t* d_mask, int32_t* d_stats, void* stream, unsigned flags = 0) {
+int run_dev(const Job& j, void* stream) {   // j: a batch in device memory
   std::lock_guard<std::mutex> lk(g_mu);
-  int rc = check_args(KIND, d1, d2, n_pairs, n, dim, metric, laf_coef, d_model, d_mask);
+  int rc = check_args(KIND, j.x1y1, j.x2y2, j.n_pairs, j.n, j.dim, j.metric, j.laf_coef, j.model_out, j.mask_out);
   if (rc) return rc;
   rc = ensure_device();
   if (rc) return rc;
-  Job j;
-  j.d1 = d1; j.d2 = d2; j.d_offsets = d_offsets; j.n_pairs = n_pairs; j.n = n; j.dim = dim;
-  j.px_th = px_th; j.conf = conf; j.laf_coef = laf_coef; j.max_iters = max_iters; j.metric = metric;
-  j.sym_check = sym_check; j.degen = degen; j.flags = flags; j.d_seeds = (const unsigned long long*)d_seeds;
-  j.d_model = d_model; j.d_mask = d_mask; j.d_stats = d_stats;
   return launch<KIND>(j, (cudaStream_t)stream);
 }
 
@@ -604,114 +511,152 @@ int run_dev(const double* d1, const double* d2, const int32_t* d_offsets, int n_
 
 extern "C" {
 
-int dgb200_find_fundamental_batch(const double* x1y1, const double* x2y2, int n_pairs, int n, int dim, double px_th,
-                                  double conf, int max_iters, int error_type, int sym_check, double laf_coef,
-                                  int degen_check, const uint64_t* seeds, double* F_out, uint8_t* mask_out,
-                                  int32_t* stats_out) {
-  return run_host<0>(x1y1, x2y2, nullptr, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef,
-                     degen_check, seeds, F_out, mask_out, stats_out);
-}
-int dgb200_find_homography_batch(const double* x1y1, const double* x2y2, int n_pairs, int n, int dim, double px_th,
-                                 double conf, int max_iters, int error_type, int sym_check, double laf_coef,
-                                 const uint64_t* seeds, double* H_out, uint8_t* mask_out, int32_t* stats_out) {
-  return run_host<1>(x1y1, x2y2, nullptr, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef, 0,
-                     seeds, H_out, mask_out, stats_out);
-}
 int dgb200_find_fundamental_batch_ex(const double* x1y1, const double* x2y2, int n_pairs, int n, int dim, double px_th,
                                      double conf, int max_iters, int error_type, int sym_check, double laf_coef,
                                      int degen_check, const uint64_t* seeds, double* F_out, uint8_t* mask_out,
                                      int32_t* stats_out, unsigned flags) {
-  return run_host<0>(x1y1, x2y2, nullptr, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef,
-                     degen_check, seeds, F_out, mask_out, stats_out, flags);
+  Job j;
+  j.x1y1 = x1y1; j.x2y2 = x2y2; j.n_pairs = n_pairs; j.n = n; j.dim = dim; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.metric = error_type; j.sym_check = sym_check; j.laf_coef = laf_coef; j.seeds = seeds;
+  j.model_out = F_out; j.mask_out = mask_out; j.stats_out = stats_out;
+  j.degen = degen_check; j.flags = flags;
+  return run_host<0>(j);
 }
 int dgb200_find_homography_batch_ex(const double* x1y1, const double* x2y2, int n_pairs, int n, int dim, double px_th,
                                     double conf, int max_iters, int error_type, int sym_check, double laf_coef,
                                     const uint64_t* seeds, double* H_out, uint8_t* mask_out, int32_t* stats_out,
                                     unsigned flags) {
-  return run_host<1>(x1y1, x2y2, nullptr, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef, 0,
-                     seeds, H_out, mask_out, stats_out, flags);
+  Job j;
+  j.x1y1 = x1y1; j.x2y2 = x2y2; j.n_pairs = n_pairs; j.n = n; j.dim = dim; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.metric = error_type; j.sym_check = sym_check; j.laf_coef = laf_coef; j.seeds = seeds;
+  j.model_out = H_out; j.mask_out = mask_out; j.stats_out = stats_out;
+  j.flags = flags;
+  return run_host<1>(j);
+}
+int dgb200_find_fundamental_batch(const double* x1y1, const double* x2y2, int n_pairs, int n, int dim, double px_th,
+                                  double conf, int max_iters, int error_type, int sym_check, double laf_coef,
+                                  int degen_check, const uint64_t* seeds, double* F_out, uint8_t* mask_out,
+                                  int32_t* stats_out) {
+  return dgb200_find_fundamental_batch_ex(x1y1, x2y2, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check,
+                                          laf_coef, degen_check, seeds, F_out, mask_out, stats_out, 0);
+}
+int dgb200_find_homography_batch(const double* x1y1, const double* x2y2, int n_pairs, int n, int dim, double px_th,
+                                 double conf, int max_iters, int error_type, int sym_check, double laf_coef,
+                                 const uint64_t* seeds, double* H_out, uint8_t* mask_out, int32_t* stats_out) {
+  return dgb200_find_homography_batch_ex(x1y1, x2y2, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check,
+                                         laf_coef, seeds, H_out, mask_out, stats_out, 0);
 }
 int dgb200_find_fundamental_batch_dev_ex(const double* d_x1y1, const double* d_x2y2, int n_pairs, int n, int dim,
                                          double px_th, double conf, int max_iters, int error_type, int sym_check,
                                          double laf_coef, int degen_check, const uint64_t* d_seeds, double* d_F_out,
                                          uint8_t* d_mask_out, int32_t* d_stats_out, void* stream, unsigned flags) {
-  return run_dev<0>(d_x1y1, d_x2y2, nullptr, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef,
-                    degen_check, d_seeds, d_F_out, d_mask_out, d_stats_out, stream, flags);
+  Job j;
+  j.x1y1 = d_x1y1; j.x2y2 = d_x2y2; j.n_pairs = n_pairs; j.n = n; j.dim = dim; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.metric = error_type; j.sym_check = sym_check; j.laf_coef = laf_coef; j.seeds = d_seeds;
+  j.model_out = d_F_out; j.mask_out = d_mask_out; j.stats_out = d_stats_out;
+  j.degen = degen_check; j.flags = flags;
+  return run_dev<0>(j, stream);
 }
 int dgb200_find_homography_batch_dev_ex(const double* d_x1y1, const double* d_x2y2, int n_pairs, int n, int dim,
                                         double px_th, double conf, int max_iters, int error_type, int sym_check,
                                         double laf_coef, const uint64_t* d_seeds, double* d_H_out, uint8_t* d_mask_out,
                                         int32_t* d_stats_out, void* stream, unsigned flags) {
-  return run_dev<1>(d_x1y1, d_x2y2, nullptr, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef, 0,
-                    d_seeds, d_H_out, d_mask_out, d_stats_out, stream, flags);
-}
-int dgb200_find_fundamental_ragged(const double* x1y1, const double* x2y2, const int32_t* offsets, int n_pairs, int dim,
-                                   double px_th, double conf, int max_iters, int error_type, int sym_check,
-                                   double laf_coef, int degen_check, const uint64_t* seeds, double* F_out,
-                                   uint8_t* mask_out, int32_t* stats_out) {
-  return run_host<0>(x1y1, x2y2, offsets, n_pairs, 0, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef,
-                     degen_check, seeds, F_out, mask_out, stats_out);
-}
-int dgb200_find_homography_ragged(const double* x1y1, const double* x2y2, const int32_t* offsets, int n_pairs, int dim,
-                                  double px_th, double conf, int max_iters, int error_type, int sym_check,
-                                  double laf_coef, const uint64_t* seeds, double* H_out, uint8_t* mask_out,
-                                  int32_t* stats_out) {
-  return run_host<1>(x1y1, x2y2, offsets, n_pairs, 0, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef, 0,
-                     seeds, H_out, mask_out, stats_out);
+  Job j;
+  j.x1y1 = d_x1y1; j.x2y2 = d_x2y2; j.n_pairs = n_pairs; j.n = n; j.dim = dim; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.metric = error_type; j.sym_check = sym_check; j.laf_coef = laf_coef; j.seeds = d_seeds;
+  j.model_out = d_H_out; j.mask_out = d_mask_out; j.stats_out = d_stats_out;
+  j.flags = flags;
+  return run_dev<1>(j, stream);
 }
 int dgb200_find_fundamental_batch_dev(const double* d_x1y1, const double* d_x2y2, int n_pairs, int n, int dim,
                                       double px_th, double conf, int max_iters, int error_type, int sym_check,
                                       double laf_coef, int degen_check, const uint64_t* d_seeds, double* d_F_out,
                                       uint8_t* d_mask_out, int32_t* d_stats_out, void* stream) {
-  return run_dev<0>(d_x1y1, d_x2y2, nullptr, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef,
-                    degen_check, d_seeds, d_F_out, d_mask_out, d_stats_out, stream);
+  return dgb200_find_fundamental_batch_dev_ex(d_x1y1, d_x2y2, n_pairs, n, dim, px_th, conf, max_iters, error_type,
+                                              sym_check, laf_coef, degen_check, d_seeds, d_F_out, d_mask_out,
+                                              d_stats_out, stream, 0);
 }
 int dgb200_find_homography_batch_dev(const double* d_x1y1, const double* d_x2y2, int n_pairs, int n, int dim,
                                      double px_th, double conf, int max_iters, int error_type, int sym_check,
                                      double laf_coef, const uint64_t* d_seeds, double* d_H_out, uint8_t* d_mask_out,
                                      int32_t* d_stats_out, void* stream) {
-  return run_dev<1>(d_x1y1, d_x2y2, nullptr, n_pairs, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef, 0,
-                    d_seeds, d_H_out, d_mask_out, d_stats_out, stream);
+  return dgb200_find_homography_batch_dev_ex(d_x1y1, d_x2y2, n_pairs, n, dim, px_th, conf, max_iters, error_type,
+                                             sym_check, laf_coef, d_seeds, d_H_out, d_mask_out, d_stats_out, stream, 0);
+}
+int dgb200_find_fundamental_ragged(const double* x1y1, const double* x2y2, const int32_t* offsets, int n_pairs, int dim,
+                                   double px_th, double conf, int max_iters, int error_type, int sym_check,
+                                   double laf_coef, int degen_check, const uint64_t* seeds, double* F_out,
+                                   uint8_t* mask_out, int32_t* stats_out) {
+  Job j;
+  j.x1y1 = x1y1; j.x2y2 = x2y2; j.n_pairs = n_pairs; j.dim = dim; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.metric = error_type; j.sym_check = sym_check; j.laf_coef = laf_coef; j.seeds = seeds;
+  j.model_out = F_out; j.mask_out = mask_out; j.stats_out = stats_out;
+  j.offsets = offsets; j.degen = degen_check;
+  return run_host<0>(j);
+}
+int dgb200_find_homography_ragged(const double* x1y1, const double* x2y2, const int32_t* offsets, int n_pairs, int dim,
+                                  double px_th, double conf, int max_iters, int error_type, int sym_check,
+                                  double laf_coef, const uint64_t* seeds, double* H_out, uint8_t* mask_out,
+                                  int32_t* stats_out) {
+  Job j;
+  j.x1y1 = x1y1; j.x2y2 = x2y2; j.n_pairs = n_pairs; j.dim = dim; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.metric = error_type; j.sym_check = sym_check; j.laf_coef = laf_coef; j.seeds = seeds;
+  j.model_out = H_out; j.mask_out = mask_out; j.stats_out = stats_out;
+  j.offsets = offsets;
+  return run_host<1>(j);
 }
 int dgb200_find_fundamental_ragged_dev(const double* d_x1y1, const double* d_x2y2, const int32_t* d_offsets, int n_pairs,
                                        int n_max, int dim, double px_th, double conf, int max_iters, int error_type,
                                        int sym_check, double laf_coef, int degen_check, const uint64_t* d_seeds,
                                        double* d_F_out, uint8_t* d_mask_out, int32_t* d_stats_out, void* stream) {
   if (!d_offsets) return fail(DGB200_E_ARG, "null offsets");
-  return run_dev<0>(d_x1y1, d_x2y2, d_offsets, n_pairs, n_max, dim, px_th, conf, max_iters, error_type, sym_check,
-                    laf_coef, degen_check, d_seeds, d_F_out, d_mask_out, d_stats_out, stream);
+  Job j;
+  j.x1y1 = d_x1y1; j.x2y2 = d_x2y2; j.n_pairs = n_pairs; j.n = n_max; j.dim = dim; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.metric = error_type; j.sym_check = sym_check; j.laf_coef = laf_coef; j.seeds = d_seeds;
+  j.model_out = d_F_out; j.mask_out = d_mask_out; j.stats_out = d_stats_out;
+  j.offsets = d_offsets; j.degen = degen_check;
+  return run_dev<0>(j, stream);
 }
 int dgb200_find_homography_ragged_dev(const double* d_x1y1, const double* d_x2y2, const int32_t* d_offsets, int n_pairs,
                                       int n_max, int dim, double px_th, double conf, int max_iters, int error_type,
                                       int sym_check, double laf_coef, const uint64_t* d_seeds, double* d_H_out,
                                       uint8_t* d_mask_out, int32_t* d_stats_out, void* stream) {
   if (!d_offsets) return fail(DGB200_E_ARG, "null offsets");
-  return run_dev<1>(d_x1y1, d_x2y2, d_offsets, n_pairs, n_max, dim, px_th, conf, max_iters, error_type, sym_check,
-                    laf_coef, 0, d_seeds, d_H_out, d_mask_out, d_stats_out, stream);
+  Job j;
+  j.x1y1 = d_x1y1; j.x2y2 = d_x2y2; j.n_pairs = n_pairs; j.n = n_max; j.dim = dim; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.metric = error_type; j.sym_check = sym_check; j.laf_coef = laf_coef; j.seeds = d_seeds;
+  j.model_out = d_H_out; j.mask_out = d_mask_out; j.stats_out = d_stats_out;
+  j.offsets = d_offsets;
+  return run_dev<1>(j, stream);
 }
 int dgb200_find_fundamental(const double* x1y1, const double* x2y2, int n, int dim, double px_th, double conf,
                             int max_iters, int error_type, int sym_check, double laf_coef, int degen_check,
                             uint64_t seed, double* F_out, uint8_t* mask_out, int32_t* stats_out) {
-  return run_host<0>(x1y1, x2y2, nullptr, 1, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef, degen_check,
-                     &seed, F_out, mask_out, stats_out);
+  return dgb200_find_fundamental_batch(x1y1, x2y2, 1, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef,
+                                       degen_check, &seed, F_out, mask_out, stats_out);
 }
 int dgb200_find_homography(const double* x1y1, const double* x2y2, int n, int dim, double px_th, double conf,
                            int max_iters, int error_type, int sym_check, double laf_coef, uint64_t seed, double* H_out,
                            uint8_t* mask_out, int32_t* stats_out) {
-  return run_host<1>(x1y1, x2y2, nullptr, 1, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef, 0, &seed,
-                     H_out, mask_out, stats_out);
+  return dgb200_find_homography_batch(x1y1, x2y2, 1, n, dim, px_th, conf, max_iters, error_type, sym_check, laf_coef,
+                                      &seed, H_out, mask_out, stats_out);
 }
 
+// u10 rows (x', y', a', b', c', x, y, a, b, c): both halves of a correspondence come from the one array
 int dgb200_find_homography_2el_batch(const double* u10, int n_pairs, int n, double px_th, double conf, int max_iters,
                                      const uint64_t* seeds, double* H_out, uint8_t* mask_out, int32_t* stats_out) {
-  return run_host<2>(u10, u10, nullptr, n_pairs, n, 10, px_th, conf, max_iters, 0, 0, 0.0, 0, seeds, H_out, mask_out,
-                     stats_out);
+  Job j;
+  j.x1y1 = u10; j.x2y2 = u10; j.n_pairs = n_pairs; j.n = n; j.dim = 10; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.seeds = seeds; j.model_out = H_out; j.mask_out = mask_out; j.stats_out = stats_out;
+  return run_host<2>(j);
 }
 int dgb200_find_homography_2el_batch_dev(const double* d_u10, int n_pairs, int n, double px_th, double conf,
                                          int max_iters, const uint64_t* d_seeds, double* d_H_out, uint8_t* d_mask_out,
                                          int32_t* d_stats_out, void* stream) {
-  return run_dev<2>(d_u10, d_u10, nullptr, n_pairs, n, 10, px_th, conf, max_iters, 0, 0, 0.0, 0, d_seeds, d_H_out,
-                    d_mask_out, d_stats_out, stream);
+  Job j;
+  j.x1y1 = d_u10; j.x2y2 = d_u10; j.n_pairs = n_pairs; j.n = n; j.dim = 10; j.px_th = px_th; j.conf = conf;
+  j.max_iters = max_iters; j.seeds = d_seeds; j.model_out = d_H_out; j.mask_out = d_mask_out; j.stats_out = d_stats_out;
+  return run_dev<2>(j, stream);
 }
 
 int dgb200_version(void) { return 2; }

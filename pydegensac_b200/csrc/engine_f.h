@@ -6,7 +6,7 @@
 //   WAVE   (parallel, speculative)  a chunk of iterations is hypothesised at once: one THREAD draws the
 //          Philox sample, solves the 7-point problem in registers/local memory and applies the oriented
 //          epipolar test; surviving models are queued and one WARP per model scores them over all
-//          correspondences in shared memory (lane-strided, shuffle reduction).  Only models whose MSAC
+//          correspondences of the FP32 tile (lane-strided, shuffle reduction).  Only models whose MSAC
 //          score can beat the running thresholds survive the wave.
 //   REPLAY (ordered, exact)         survivors are re-evaluated in iteration order with the reference's
 //          control flow: so-far-the-best bookkeeping, symmetric gate, LO scheduling (first-50 rule),

@@ -30,7 +30,7 @@ namespace dg {
 struct alignas(16) Pt32 { float u, v, s, t; };   // (x1 - c1x, y1 - c1y, x2 - c2x, y2 - c2y)
 
 struct Tile32 {
-  const Pt32* pts;    // centred single-precision correspondences (shared memory when they fit)
+  const Pt32* pts;    // centred single-precision correspondences (in the CTA's slab)
   double cen[4];      // centroids c1x, c1y, c2x, c2y
   double bnd[4];      // max |u|, |v|, |s|, |t|
 };

@@ -24,8 +24,8 @@ DG_HD size_t workspace_bytes(int N, int chunk, bool laf) {
   b += align_up(sizeof(int) * (size_t)chunk, 128);                // survivors
   b += align_up(sizeof(double) * 16 * (size_t)chunk, 128);        // null-space bases of the wave
   b += align_up(sizeof(uint32_t) * kHashCap, 128) * 3;            // hash table
-  b += align_up(sizeof(double) * (size_t)N, 128) * 4;             // SoA correspondences when not in smem
-  b += align_up(16 * ((size_t)N + 1), 128);                       // FP32 filter tile when not in smem (pair-interleaved, N+1 slots)
+  b += align_up(sizeof(double) * (size_t)N, 128) * 4;             // SoA correspondences of the pair
+  b += align_up(16 * ((size_t)N + 1), 128);                       // FP32 filter tile (pair-interleaved, N+1 slots)
   return b;
 }
 
